@@ -7,7 +7,7 @@ candidate allocations per step per GPU (synthetic fleet, SURVEY.md §8d, PCG64 s
 One step = one pass of the hot path over that grid: state-dependent M/M/1/K evaluation
 of every cell + SLO feasibility + cost + transition penalty + per-model argmin.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun, one rank per GPU: the fleet is sharded by model (weak
 scaling: 100 models per GPU), the only exchange is ONE NCCL all-gather of the per-shard
@@ -35,6 +35,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "candidate allocations/sec"
 UNIT = "candidates/s"
@@ -59,7 +60,15 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary BASELINE configurations")
     ap.add_argument("--ref-seconds", type=float, default=90.0,
                     help="--impl reference: the per-step sample is sized so that the whole run takes about this long")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl ours: after the timed steps, write the winner records of the last timed step as "
+                         "DIR/winner_<column>.npy (integer columns as float64, float columns as float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def workload(rank: int):
@@ -237,7 +246,7 @@ def cpu_baseline_port(n_pairs: int, reps: int = 5) -> dict:
     import multiprocessing as mp
 
     import oracle
-    oracle.build()
+    oracle.lib()  # loaded before the workers fork; build() compiled it
     pairs = sample_pairs(n_pairs)
     cpu = sorted(os.sched_getaffinity(0))[0]
     ctx = mp.get_context("fork")
@@ -263,7 +272,7 @@ def run_reference(args):
     import multiprocessing as mp
 
     import oracle
-    oracle.build()
+    oracle.lib()  # loaded before the workers fork; build() compiled it
     cores = len(os.sched_getaffinity(0))  # every logical CPU the process may use
     quota = cpu_quota_cores()            # ... unless a cgroup quota caps the CPU time below that
     per_pair = N_BATCH * N_REPLICAS
@@ -333,7 +342,6 @@ def extras_single_gpu(eng) -> dict:
     import oracle
     from workload_variant_autoscaler_b200 import synth_fleet
     from workload_variant_autoscaler_b200.fleet import CONFIG1_LOADS, config1_fleet
-    oracle.build()
     out = {}
 
     # configs[0]: the single VariantAutoscaling of the emulator sample (one candidate, N = 4): latency per reconcile
@@ -451,6 +459,17 @@ def extras_sharded(eng, rank, world, dev) -> dict:
 # ----------------------------------------------------------------------------
 # GPU leg
 # ----------------------------------------------------------------------------
+def dump_winners(block: np.ndarray, n_servers: int, out_dir: str) -> None:
+    """One device winner block (int32 [10 * S]: a slot of S words per column of ALLOC_COLUMNS, the feasible flags in
+    the first S bytes of theirs) -> out_dir/winner_<column>.npy, integer columns widened to float64 (exact)."""
+    from workload_variant_autoscaler_b200._abi import ALLOC_COLUMNS
+    os.makedirs(out_dir, exist_ok=True)
+    slots = block.reshape(len(ALLOC_COLUMNS), n_servers)
+    for k, (name, dt) in enumerate(ALLOC_COLUMNS):
+        col = slots[k].view(np.uint8)[:n_servers] if dt is np.uint8 else slots[k].view(dt)
+        np.save(os.path.join(out_dir, f"winner_{name}.npy"), col if dt is np.float32 else col.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -652,6 +671,8 @@ def run_ours(args):
         dist.barrier()
     wall = time.perf_counter() - wall0
     launches = eng.launch_count - launches0
+    if args.dump_outputs and rank == 0:  # the block the last timed step wrote (overlapped steps alternate two)
+        dump_winners(blocks[(step_no[0] - 1) & 1 if overlap else 0][0].cpu().numpy(), S, args.dump_outputs)
     total_ms = torch.tensor([sum(per_step)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)

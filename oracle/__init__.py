@@ -77,7 +77,8 @@ def lib():
     global _lib
     if _lib is not None:
         return _lib
-    build()
+    if not os.path.exists(_SO):  # a stale library is rebuilt by build(), not here: bench.py may run on a read-only tree
+        build()
     L = C.CDLL(_SO)
     f, i, vp = C.c_float, C.c_int, C.c_void_p
     L.wvao_prefill_time.restype = f

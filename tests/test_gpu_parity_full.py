@@ -204,7 +204,7 @@ def _peer_worker(rank, world, port, out_dir):
 def test_peer_exchange_matches_nccl(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs on one box (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs on one machine")
     import torch.multiprocessing as tmp_mp
     world = 2
     tmp_mp.spawn(_peer_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
@@ -260,7 +260,7 @@ def _sharded_worker(rank, world, port, out_dir):
 def test_sharded_solves_on_two_gpus_match_the_oracle(tmp_path):
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs on one box (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs on one machine")
     import torch.multiprocessing as tmp_mp
     world = 2
     tmp_mp.spawn(_sharded_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
