@@ -165,6 +165,9 @@ struct wva_handle {
     bool dbg_cycles = false;
     const unsigned* dbg_plan = nullptr;
     size_t dbg_n = 0;
+    const int* dbg_row_j = nullptr;  // row_j / row_res of the last grid solve (wva_dbg_read_rows)
+    const uint8_t* dbg_row_res = nullptr;
+    size_t dbg_rows_n = 0;
     PinBuf out_stage;
 
     int fail(int code, const char* what, cudaError_t e = cudaSuccess) {
@@ -837,11 +840,19 @@ int prepare_grid(wva_handle* h, const wva_grid* grid, GridPlan* plan) {
     CK(h->d_best.ensure(sizeof(int) * n_best));
     g.best_rank = (int*)h->d_best.p;
     const size_t n_pairs_alloc = std::max<size_t>((size_t)S * A, 1);
-    CK(h->d_rows.ensure(align_up((2 * sizeof(double) + sizeof(int)) * n_best + 64) + 48 * n_pairs_alloc));
+    const size_t rows_bytes = align_up((2 * sizeof(double) + sizeof(int)) * n_best + 64);
+    CK(h->d_rows.ensure(rows_bytes + align_up(48 * n_pairs_alloc) + n_best));
     g.row_acc = (double*)h->d_rows.p;
     g.row_sump = g.row_acc + n_best;
     g.row_j = (int*)(g.row_sump + n_best);
-    g.pair_rec = (float4*)((char*)h->d_rows.p + align_up((2 * sizeof(double) + sizeof(int)) * n_best + 64));
+    g.pair_rec = (float4*)((char*)h->d_rows.p + rows_bytes);
+    g.row_res = (uint8_t*)h->d_rows.p + rows_bytes + align_up(48 * n_pairs_alloc);
+    h->dbg_row_j = g.row_j;
+    h->dbg_row_res = g.row_res;
+    h->dbg_rows_n = (size_t)S * A * R;
+    // row resolution (DESIGN §3.2b); WVA_GRID_ROWRES=0 keeps the per-cell evaluation of every shared cell
+    g.row_resolve = 1;
+    if (const char* e = getenv("WVA_GRID_ROWRES")) g.row_resolve = atoi(e) != 0;
     g.Bmax = h->grid_Bmax;
     g.fb_count = (int*)h->d_ctrl.p + CTRL_FB_COUNT;
     g.fb_cap = (int)std::min<size_t>(nc, (size_t)1 << 22);
@@ -1945,6 +1956,15 @@ long long wva_dbg_read_size(wva_handle* h, unsigned* out4, long long cap) {  // 
     if (!h || !h->d_dbg.p) return 0;
     const long long n = std::min<long long>((long long)h->dbg_n, cap);
     cudaMemcpy(out4, h->d_dbg.p, 16 * n, cudaMemcpyDeviceToHost);
+    return n;
+}
+// Per (server, accelerator, replica level) of the last grid solve: the shared chain's last state (INT_MAX: none) and
+// whether grid_rows resolved the row (§3.2b).  Returns the number of rows copied.
+long long wva_dbg_read_rows(wva_handle* h, int* row_j, uint8_t* row_res, long long cap) {
+    if (!h || !h->dbg_row_j) return 0;
+    const long long n = std::min<long long>((long long)h->dbg_rows_n, cap);
+    cudaMemcpy(row_j, h->dbg_row_j, sizeof(int) * n, cudaMemcpyDeviceToHost);
+    cudaMemcpy(row_res, h->dbg_row_res, n, cudaMemcpyDeviceToHost);
     return n;
 }
 long long wva_dbg_read_cycles(wva_handle* h, unsigned* cycles, unsigned* cells, long long cap) {

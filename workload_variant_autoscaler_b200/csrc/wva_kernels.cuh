@@ -329,6 +329,8 @@ struct GridArgs {
     double* row_acc;                // [S*A*R] shared-chain results per (server, accelerator, replica)
     double* row_sump;
     int* row_j;                     // last state of the shared chain (INT_MAX: no sharing)
+    uint8_t* row_res;               // 1: grid_rows resolved the row's shared cells into best_rank (§3.2b)
+    int row_resolve;                // 0: row resolution off (WVA_GRID_ROWRES=0)
     int Bmax;                       // table length
     long long n_cells;
     unsigned* order;         // [n_cells] cell ids, sorted by length class inside each chunk of kSortChunk cells
@@ -430,6 +432,15 @@ __device__ __forceinline__ bool cell_feasible(const FeasRow& fr, int r, float la
     if (fr.tps) feas = feas && (lambda <= fr.lim);
     return feas;
 }
+// Analyze's rate checks for a cell of a pair that has a table (queueanalyzer.go:135-143): a positive rate inside the
+// stability range of the batch size (rmax = RateRange.Max), and a queue of at least two states (K = b + b * ratio).
+__device__ __forceinline__ bool cell_analysable(float rate, float rmax, int K) {
+    return !(rate <= 0.0f) && !(rate > rmax) && K >= 2;
+}
+// The cell's chain is its row's shared chain (§3.2a): the row has one (jl != INT_MAX) and the batch size is past it.
+__device__ __forceinline__ bool cell_shared(int jl, int b, int K) {
+    return jl != INT_MAX && b >= jl + 2 && K < (1 << 23);
+}
 __device__ __forceinline__ void store_cell(const GridArgs& g, long long cell, int ok, int feas, const Metrics& m) {
     g.cells.flags[cell] = (uint8_t)(ok | (feas << 1));
     g.cells.ttft[cell] = m.ttft;
@@ -526,10 +537,62 @@ __device__ __forceinline__ Metrics shared_cell_metrics_inv(const PairConst& pc, 
     return m;
 }
 
+// Row resolution (DESIGN §3.2b).  On an invariant row a shared cell depends on its batch size N only through
+// eff = min(effu, N), which does not decrease as N grows.  With the operands below finite, beta >= 0 and d_in >= 0 (or
+// no input tokens), itl = RN(alpha + RN(beta eff)) and ttft = RN(w0 + RN(gamma + RN(d_in eff))) do not decrease either
+// (RN is monotone), so the SLO part of cell_feasible holds for a prefix of the batch sizes.  Everything else a shared
+// cell's feasibility depends on is a function of the batch size alone (row_gate).  Hence the smallest feasible shared
+// rank of the row is the first rank that passes row_gate if the SLO test holds there, and there is none otherwise.
+__device__ __forceinline__ bool row_monotone(const PairConst& pc, const RowInv& ri) {
+    const bool prefill = pc.in_zero || (isfinite(pc.d_in) && pc.d_in >= 0.0f);
+    return isfinite(pc.alpha) && isfinite(pc.beta) && pc.beta >= 0.0f && isfinite(pc.gamma) && prefill &&
+           isfinite(ri.w0) && isfinite(ri.effu);
+}
+// The conditions under which a cell of the row is analysed as a shared cell, plus the TPS stability limit of its
+// feasibility: the parts that depend on the batch size and not on the chain.
+__device__ __forceinline__ bool row_gate(float rate, float lambda, bool tps, float rmax, int jl, int b, int K) {
+    return cell_analysable(rate, rmax, K) && cell_shared(jl, b, K) && (!tps || lambda <= feas_lim(rmax));
+}
+
 // One CTA per (server, accelerator) pair, one lane per replica level: the chain every large-enough
 // batch size shares.  The pair's table is staged in shared memory first (coalesced), so the serial
 // chains read it at shared-memory latency instead of waiting for L2 on every step.
 constexpr int kRowsSmemEntries = 1536;  // 48 KB of 32-byte entries; longer tables are read from global
+
+// The smallest feasible batch rank among the shared cells of a row that row_monotone admits (INT_MAX: none), t = the
+// pair's table index.  A row whose cells all fail row_gate scans every rank, so the loads go four ranks at a time.
+__device__ __forceinline__ int resolve_row(const GridArgs& g, int t, float rate, float lambda, FeasRow fr, int rep,
+                                           const PairConst& pc, const RowInv& inv, int jl) {
+    const int B = g.B;
+    int lo = 0, hi = B;  // first rank with a batch size past the shared chain (ranks ascend with the batch size)
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (g.batch[g.rank_to_bi[mid]] >= jl + 2) hi = mid; else lo = mid + 1;
+    }
+    const float* rmax = (const float*)(g.pb + (size_t)t * B);  // component x of the (table, batch) constants
+    for (int r0 = lo; r0 < B; r0 += 4) {
+        int bi[4], b[4];
+        float rm[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) bi[u] = g.rank_to_bi[min(r0 + u, B - 1)];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            b[u] = g.batch[bi[u]];
+            rm[u] = rmax[4 * bi[u]];
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int K = b[u] + b[u] * g.f.ratio;
+            if (r0 + u < B && row_gate(rate, lambda, fr.tps, rm[u], jl, b[u], K)) {
+                fr.lim = feas_lim(rm[u]);
+                const Metrics m = shared_cell_metrics_inv(pc, inv, lambda, b[u], false);
+                return cell_feasible(fr, rep, lambda, m) ? r0 + u : INT_MAX;
+            }
+        }
+    }
+    return INT_MAX;
+}
+
 __global__ void __launch_bounds__(128) grid_rows(GridArgs g) {
     extern __shared__ double rows_tab[];
     const DevFleet& f = g.f;
@@ -577,18 +640,26 @@ __global__ void __launch_bounds__(128) grid_rows(GridArgs g) {
         l2s0 = log2f((float)tab[0]);
         ls_end = (g.ls + toff + g.pair_tab_idx[sa])[g.Bmax - 1];
     }
+    // row resolution (§3.2b) only when the caller does not want the cell table: grid_sort_local then never visits the
+    // shared cells of a resolved row
+    const bool resolve = toff >= 0 && g.row_resolve && !g.want_cells;
+    PairConst pc{};
+    FeasRow fr{};
+    if (resolve) {
+        pc = pair_const(qparams_of(f, s, sa - s * f.A));
+        fr = feas_row(f, s, 0.0f);
+    }
     for (int ri = threadIdx.x; ri < g.R; ri += blockDim.x) {
         const size_t row = (size_t)sa * g.R + ri;
         int j = INT_MAX;
         double acc = 0.0, sump = 0.0;
         // per-replica rate, lambda and log2(lambda) of the server (rate = total / replicas, lambda = rate / 1000): every pair CTA
         // derives its own copy, the CTA of accelerator 0 publishes it for the later kernels; the
-        // (pair, replica) slot of the batch-rank minimum is reset here too
+        // (pair, replica) slot of the batch-rank minimum is reset here too (or set to the resolved row's minimum)
         const float rate = __fdiv_rn(total_rate_of(f, s), (float)g.replicas[ri]);
         const float lambda = __fdiv_rn(rate, 1000.0f);
         const float4 rt = make_float4(rate, lambda, log2f(lambda), 0.0f);
         if (sa == s * f.A) g.rt[s * g.R + ri] = rt;
-        g.best_rank[row] = INT_MAX;
         if (toff >= 0 && rt.x > 0.0f) {
             // skip rows whose chain is (by the log-domain estimate) still far from negligible at the end of
             // the table: they cannot be shared and would only burn Bmax steps to find that out
@@ -600,6 +671,18 @@ __global__ void __launch_bounds__(128) grid_rows(GridArgs g) {
                 if (ok) j = jl;
             }
         }
+        int best = INT_MAX;
+        uint8_t res = 0;
+        if (resolve && j != INT_MAX) {
+            RowInv inv;
+            if (row_invariant(pc, acc, __dsub_rn(1.0, sump), row_resp_time(acc, lambda), lambda, g.Bmax, inv) &&
+                row_monotone(pc, inv)) {
+                res = 1;
+                best = resolve_row(g, g.pair_tab_idx[sa], rt.x, lambda, fr, g.replicas[ri], pc, inv, j);
+            }
+        }
+        g.best_rank[row] = best;
+        g.row_res[row] = res;
         g.row_j[row] = j;
         g.row_acc[row] = acc;
         g.row_sump[row] = sump;
@@ -633,13 +716,16 @@ __device__ __forceinline__ unsigned seg_inc(unsigned* counters, int key) {
 // items globally, so the launch is longest-first while a pair's cells stay adjacent.
 __device__ __forceinline__ void grid_items_plan(const GridArgs& g);
 __global__ void __launch_bounds__(kSortThreads, 2) grid_sort_local(GridArgs g) {
-    __shared__ uint8_t keys[kSortChunk];
+    __shared__ __align__(16) uint8_t keys[kSortChunk];
     __shared__ uint8_t sorted_keys[kSortChunk];
     __shared__ unsigned hist[kClasses];
     __shared__ unsigned cursor[kClasses];
     __shared__ unsigned item_base;
     const DevFleet& f = g.f;
     if (threadIdx.x < kClasses) hist[threadIdx.x] = 0;
+    // every key starts as class 255 (not analysable, or finished here): the walk stores only the other classes
+    static_assert(kSortChunk == 16 * kSortThreads, "one 16-byte store per thread fills the keys");
+    reinterpret_cast<uint4*>(keys)[threadIdx.x] = make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
     __syncthreads();
     const long long base = (long long)blockIdx.x * kSortChunk;
     const int n_here = (int)min((long long)kSortChunk, g.n_cells - base);
@@ -661,15 +747,18 @@ __global__ void __launch_bounds__(kSortThreads, 2) grid_sort_local(GridArgs g) {
         };
         // pair-level constants are re-read only when the walk crosses into the next pair; so are the
         // lane's own row constants (its first two replica levels: rate, lambda, the row's shared chain)
+        // what a lane knows about the shared cells of its row: evaluated per cell (general or invariant form), or
+        // already resolved into best_rank by grid_rows (§3.2b)
+        enum : uint8_t { kRowCells = 0, kRowInv = 1, kRowResolved = 2 };
         struct LaneRow {
             float4 rt;
-            // shared-chain results of the row.  inv == false: a = sum(i p[i]), b = 1 - sumP, r = resp (avgNumInSystem /
-            // throughput).  inv == true (row_invariant holds): the three floats of RowInv ride in the same registers
-            // (a = {f0, w0}, r = effu), so the hot loop carries no more state than before.
+            // shared-chain results of the row.  kRowCells: a = sum(i p[i]), b = 1 - sumP, r = resp (avgNumInSystem /
+            // throughput).  kRowInv (row_invariant holds): the three floats of RowInv ride in the same registers
+            // (a = {f0, w0}, r = effu), so the hot loop carries no more state than before.  kRowResolved: unused.
             double a, b;
             float r;
             int jl, rep;
-            bool inv;
+            uint8_t kind;
         };
         LaneRow c0{}, c1{};
         unsigned sa = (row0 + warp) / B;
@@ -683,14 +772,15 @@ __global__ void __launch_bounds__(kSortThreads, 2) grid_sort_local(GridArgs g) {
             const size_t rowid = (size_t)sa * R + ri;
             c.rt = g.rt[(unsigned)s * R + ri];
             c.jl = g.row_j[rowid];
+            c.kind = g.row_res[rowid] ? kRowResolved : kRowCells;
+            if (c.kind == kRowResolved) return;
             c.a = g.row_acc[rowid];
             c.b = __dsub_rn(1.0, g.row_sump[rowid]);
             c.r = row_resp_time(c.a, c.rt.y);
             c.rep = g.replicas[ri];
-            c.inv = false;
             RowInv inv;
             if (c.jl != INT_MAX && row_invariant(pc, c.a, c.b, c.r, c.rt.y, g.Bmax, inv)) {
-                c.inv = true;
+                c.kind = kRowInv;
                 c.a = __hiloint2double(__float_as_int(inv.w0), __float_as_int(inv.f0));
                 c.r = inv.effu;
             }
@@ -715,22 +805,28 @@ __global__ void __launch_bounds__(kSortThreads, 2) grid_sort_local(GridArgs g) {
             }
             const int b = g.batch[bi];
             const int K = b + b * f.ratio;
+            // a cell that is key 255 without any work: outside the chunk, no table, or one that would share the chain
+            // of a resolved row (then it is either shared and already in best_rank, or not analysable)
+            auto idle = [&](unsigned ri, const LaneRow& c) {
+                const long long cell = (long long)row * R + ri;
+                return ri >= R || cell < base || cell >= base + n_here || toff < 0 ||
+                       (c.kind == kRowResolved && cell_shared(c.jl, b, K));
+            };
+            if (R <= 64 && __all_sync(0xffffffffu, idle(lane, c0) && idle(lane + 32, c1))) continue;
             float4 pb = make_float4(0.f, 0.f, 0.f, 0.f);
             if (toff >= 0) pb = g.pb[(size_t)t * g.B + bi];
             if (fr.tps) fr.lim = feas_lim(pb.x);
             const int rank = g.batch_rank[bi];
             // one cell: (row, ri) with the lane's cached row constants
             auto do_cell = [&](unsigned ri, const LaneRow& c, int slot) {
-                const long long cell = (long long)row * R + ri;
-                if (cell < base || cell >= base + n_here) return;
+                if (idle(ri, c)) return;
                 int key = 255;
-                bool done_here = false;
-                if (toff >= 0 && !(c.rt.x <= 0.0f) && !(c.rt.x > pb.x) && K >= 2) {  // Analyze: queueanalyzer.go:135-143
-                    if (c.jl != INT_MAX && b >= c.jl + 2 && K < (1 << 23)) {
-                        done_here = true;
+                if (cell_analysable(c.rt.x, pb.x, K)) {  // Analyze: queueanalyzer.go:135-143
+                    if (cell_shared(c.jl, b, K)) {
                         // the whole solve is shared with the row: only the N-dependent tail is per cell
+                        const long long cell = (long long)row * R + ri;
                         Metrics m;
-                        if (c.inv) {
+                        if (c.kind == kRowInv) {
                             RowInv inv;
                             inv.f0 = __int_as_float(__double2loint(c.a));
                             inv.w0 = __int_as_float(__double2hiint(c.a));
@@ -750,8 +846,10 @@ __global__ void __launch_bounds__(kSortThreads, 2) grid_sort_local(GridArgs g) {
                         key = length_class(estimate_len(g.tab + 4 * toff, g.ls + toff + t, b, K, c.rt.y, c.rt.z, pb.w, pb.y, pb.z));
                     }
                 }
-                keys[cell - base] = (uint8_t)key;
-                if (key != 255) seg_inc(hist, key);  // class 255 (finished here / not analysable) needs no slot
+                if (key != 255) {  // class 255 (finished here / not analysable) needs no slot and keeps its key
+                    keys[(long long)row * R + ri - base] = (uint8_t)key;
+                    seg_inc(hist, key);
+                }
                 // (the cell table, when requested, is cleared by the host before the launch: cells that are never
                 // analysed read back as 0 without a store per cell here)
             };
@@ -1223,8 +1321,9 @@ __global__ void __launch_bounds__(256) grid_finalize(GridArgs g, AllocCols winne
                 const long long cell = ((long long)row / g.R * g.B + k.bi) * g.R + ri;
                 const int jl = g.row_j[row];
                 const int K = b + b * f.ratio;
-                if (!g.want_cells && jl != INT_MAX && b >= jl + 2 && K < (1 << 23)) {
-                    // the cell shares its row's chain and was not stored: grid_sort_local's evaluation again
+                if (!g.want_cells && cell_shared(jl, b, K)) {
+                    // the cell shares its row's chain and was not stored: the evaluation grid_sort_local (or, for a
+                    // resolved row, grid_rows) ran for it, again
                     const float lambda = g.rt[s * g.R + ri].y;
                     ModelStats st;
                     stats_from_row(g.row_acc[row], g.row_sump[row], b, lambda, st);
