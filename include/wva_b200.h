@@ -170,7 +170,10 @@ typedef struct wva_cells {
 /* Latency sweep (BASELINE config 3): for each (server, accelerator) pair,
  * Analyze at n_rates rates linearly spaced in [RateRange.Min, RateRange.Max*0.999].
  * Output index = (s*A + a)*n_rates + i. valid = 0 where the pair has no model or
- * Analyze returned an error. */
+ * Analyze returned an error.  Points whose chain leaves the streaming solve's numeric
+ * window (including those the reference rescales) are re-run on the stored-vector
+ * fallback; WVA_ERR_UNSUPPORTED only where the reference's rescale would not
+ * terminate or more than 2^22 points need the fallback. */
 typedef struct wva_sweep_out {
     uint8_t *valid;
     float *rate;       /* req/sec                                                  */

@@ -168,6 +168,7 @@ struct wva_handle {
     const int* dbg_row_j = nullptr;  // row_j / row_res of the last grid solve (wva_dbg_read_rows)
     const uint8_t* dbg_row_res = nullptr;
     size_t dbg_rows_n = 0;
+    int dbg_fb_count = 0;  // solves of the last call that took the stored-vector fallback (wva_dbg_fallback_count)
     PinBuf out_stage;
 
     int fail(int code, const char* what, cudaError_t e = cudaSuccess) {
@@ -651,6 +652,7 @@ int finish_timing(wva_handle* h) {
 }
 
 int check_fallback_status(wva_handle* h, const int* ctrl_host, long long cap) {
+    h->dbg_fb_count = ctrl_host[CTRL_FB_COUNT];  // before the cap test: a count above it is reported as well
     if (ctrl_host[CTRL_FB_STATUS] != 0)
         return h->fail(WVA_ERR_UNSUPPORTED, "input outside the supported numeric domain (rescale loop does not terminate)");
     if ((long long)ctrl_host[CTRL_FB_COUNT] > cap)
@@ -1781,6 +1783,7 @@ int wva_sweep(wva_handle* h, const wva_fleet* fleet, int32_t n_rates, wva_sweep_
     CK(cudaMemsetAsync(p, 0, std::max<size_t>(out_bytes, 256), h->stream));
     CK(cudaEventRecord(h->ev_d0, h->stream));
     CK(cudaEventRecord(h->ev_k0, h->stream));
+    long long fb_cap = 0;
     if (n) {
         CK(h->d_tab_pair.ensure(sizeof(int) * n));
         CK(h->d_tab_off.ensure(sizeof(long long) * n));
@@ -1811,6 +1814,16 @@ int wva_sweep(wva_handle* h, const wva_fleet* fleet, int32_t n_rates, wva_sweep_
         g.throughput = (float*)(p + align_up(n_out) + 3 * align_up(4 * n_out));
         g.rho = (float*)(p + align_up(n_out) + 4 * align_up(4 * n_out));
         g.fb_count = (int*)h->d_ctrl.p + CTRL_FB_COUNT;
+        fb_cap = (long long)std::min<size_t>((size_t)n * n_rates, (size_t)1 << 22);
+        g.fb_cap = (int)fb_cap;
+        CK(h->d_fb_list.ensure(sizeof(long long) * g.fb_cap));
+        g.fb_points = (long long*)h->d_fb_list.p;
+        // The fallback's scratch is sized for the longest chain before the launch, as the grid and size paths do:
+        // 128 slots of (K + 1) doubles, about 12 GB at N = 2^20 with the default queue ratio, kept by the handle.
+        size_t slot_doubles;
+        int Kmax;
+        rc = ensure_scratch(h, lens[0], hf.tun.max_queue_to_batch_ratio, &slot_doubles, &Kmax);  // lens: descending
+        if (rc) return rc;
         int per_sm = 0;
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, sweep_kernel, 256, 0));
         per_sm = std::max(1, std::min(per_sm, 8));
@@ -1818,10 +1831,14 @@ int wva_sweep(wva_handle* h, const wva_fleet* fleet, int32_t n_rates, wva_sweep_
         unsigned blocks = std::min<unsigned>((unsigned)(h->sm_count * per_sm), (items + 7) / 8);
         CK(cudaEventRecord(h->ev_k0, h->stream));
         sweep_kernel<<<blocks, 256, 0, h->stream>>>(g);
-        h->launches++;
+        CK(cudaEventRecord(h->ev_k1, h->stream));
+        sweep_fallback<<<kFbBlocks, kFbThreads, 0, h->stream>>>(g, (double*)h->d_scratch.p, slot_doubles, Kmax,
+                                                                (int*)h->d_ctrl.p + CTRL_FB_STATUS);
+        h->launches += 2;
         CK(cudaGetLastError());
+    } else {
+        CK(cudaEventRecord(h->ev_k1, h->stream));
     }
-    CK(cudaEventRecord(h->ev_k1, h->stream));
     CK(h->out_stage.ensure(256));
     int* ctrl_host = (int*)h->out_stage.p;
     CK(cudaMemcpyAsync(ctrl_host, h->d_ctrl.p, CTRL_INTS * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
@@ -1838,9 +1855,7 @@ int wva_sweep(wva_handle* h, const wva_fleet* fleet, int32_t n_rates, wva_sweep_
     }
     rc = finish_timing(h);
     if (rc) return rc;
-    if (ctrl_host[CTRL_FB_COUNT] != 0)
-        return h->fail(WVA_ERR_UNSUPPORTED, "sweep point outside the streaming solve's numeric window");
-    return WVA_OK;
+    return check_fallback_status(h, ctrl_host, fb_cap);
 }
 
 // ---- self-check of the exact-division primitive (not part of the public ABI) ------------------
@@ -1967,6 +1982,9 @@ long long wva_dbg_read_rows(wva_handle* h, int* row_j, uint8_t* row_res, long lo
     cudaMemcpy(row_res, h->dbg_row_res, n, cudaMemcpyDeviceToHost);
     return n;
 }
+// Number of cells (grid), candidates (analyze / solve / resolve) or sweep points of the last call that left the
+// streaming solve's exponent windows and were re-run on the stored-vector fallback (-1 without a handle).
+int wva_dbg_fallback_count(wva_handle* h) { return h ? h->dbg_fb_count : -1; }
 long long wva_dbg_read_cycles(wva_handle* h, unsigned* cycles, unsigned* cells, long long cap) {
     if (!h || !h->d_dbg.p) return 0;
     const long long n = std::min<long long>((long long)h->dbg_n, cap);

@@ -11,6 +11,7 @@
 //   trivial_kernel      nil / zero-load candidates
 //   unlimited_kernel    Server.Calculate value + SolveUnlimited argmin per server
 //   sweep_kernel        Analyze over a rate sweep per (server, acc)
+//   sweep_fallback      stored-vector re-run of sweep points that bailed
 #pragma once
 #include "wva_device.cuh"
 
@@ -1722,7 +1723,9 @@ struct SweepArgs {
     unsigned* counter;
     uint8_t* valid;
     float *rate, *ttft, *itl, *throughput, *rho;
-    int* fb_count;
+    int* fb_count;         // sweep points that need the stored-vector fallback
+    long long* fb_points;  // their point indices e * n_rates + i (entry of pair_list, rate index), up to fb_cap
+    int fb_cap;
 };
 
 __global__ void __launch_bounds__(256) sweep_kernel(SweepArgs g) {
@@ -1762,7 +1765,8 @@ __global__ void __launch_bounds__(256) sweep_kernel(SweepArgs g) {
                 m = metrics_from(q, N, st);
                 ok = 1;
             } else {
-                atomicAdd(g.fb_count, 1);
+                const int k = atomicAdd(g.fb_count, 1);
+                if (k < g.fb_cap) g.fb_points[k] = (long long)e * g.n_rates + i;
             }
         }
         g.valid[o] = ok;
@@ -1771,6 +1775,46 @@ __global__ void __launch_bounds__(256) sweep_kernel(SweepArgs g) {
         g.throughput[o] = m.throughput;
         g.rho[o] = m.rho;
         }
+    }
+}
+
+// Stored-vector re-run of the sweep points sweep_kernel bailed on (p or the sum left the streaming solve's window,
+// e.g. a chain the reference rescales).  Slots as in grid_fallback; the rate is recomputed exactly as sweep_kernel
+// computed it.
+__global__ void sweep_fallback(SweepArgs g, double* scratch, size_t slot_doubles, int Kmax, int* fb_status) {
+    const DevFleet& f = g.f;
+    const int n_slots = gridDim.x * blockDim.x;
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
+    int n = *g.fb_count;
+    if (n > g.fb_cap) n = g.fb_cap;
+    double* p = scratch + (size_t)slot * slot_doubles;
+    float* sr = (float*)(p + Kmax + 1);
+    for (int k = slot; k < n; k += n_slots) {
+        const long long pt = g.fb_points[k];
+        const int e = (int)(pt / g.n_rates), i = (int)(pt % g.n_rates);
+        const int pair = g.pair_list[e];
+        const int s = pair / f.A, a = pair % f.A;
+        const int N = g.pair_N[e], K = N + N * f.ratio;
+        const double* tab = g.tab + 4 * g.tab_off[e];
+        for (int j = 0; j < N; ++j) sr[j] = (float)tab[4 * j];
+        const float rmin = rate_min_of(sr[0]), rmax = rate_max_of(sr[N - 1]);
+        const float hi = __fmul_rn(rmax, 0.999f);
+        const float span = __fsub_rn(hi, rmin);
+        const float frac = g.n_rates > 1 ? __fdiv_rn((float)i, (float)(g.n_rates - 1)) : 0.0f;
+        const float rate = __fadd_rn(rmin, __fmul_rn(span, frac));
+        ModelStats st;
+        const int rc = solve_stored(p, sr, N, K, __fdiv_rn(rate, 1000.0f), st);
+        if (rc != 0) {
+            atomicExch(fb_status, rc);
+            continue;
+        }
+        const Metrics m = metrics_from(qparams_of(f, s, a), N, st);
+        const size_t o = (size_t)pair * g.n_rates + i;
+        g.valid[o] = 1;
+        g.ttft[o] = m.ttft;
+        g.itl[o] = m.avg_token_time;
+        g.throughput[o] = m.throughput;
+        g.rho[o] = m.rho;
     }
 }
 
