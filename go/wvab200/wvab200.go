@@ -10,6 +10,7 @@
 // i.e. Server.Calculate + Manager.Optimize + System.GenerateSolution of pkg/core, pkg/manager; plus
 //   - Engine.Upload / UpdateLoad / Resolve: the streaming reconcile (fleet resident on the GPU, only the load
 //     columns travel per tick: wva_upload / wva_update_load / wva_resolve)
+//   - Engine.ResolveScenarios: Resolve under many arrival-rate scenarios in one call (wva_resolve_scenarios)
 //   - Engine.Summarize: System.AllocateByType + Solver.Solve's allocation diffs (wva_summarize).
 //   - Engine.MM1K: analyzer.MM1KModel (closed form) for arrays of (K, lambda, mu) (wva_mm1k_solve).
 // tests/c_abi/solve_smoke.c drives the same entry points from compiled C.
@@ -300,6 +301,13 @@ func newAllocs(n int, pin *runtime.Pinner) (*allocs, C.wva_allocs) {
 	return a, c
 }
 
+// slice views records lo .. hi-1 (one scenario's block of a wva_resolve_scenarios result).
+func (a *allocs) slice(lo, hi int) *allocs {
+	return &allocs{feasible: a.feasible[lo:hi], acc: a.acc[lo:hi], replicas: a.replicas[lo:hi], batch: a.batch[lo:hi],
+		cost: a.cost[lo:hi], value: a.value[lo:hi], itl: a.itl[lo:hi], ttft: a.ttft[lo:hi], rho: a.rho[lo:hi],
+		maxRate: a.maxRate[lo:hi]}
+}
+
 func (e *Engine) fail(what string, rc C.int) error {
 	return fmt.Errorf("%s: %s: %s", what, C.GoString(C.wva_strerror(rc)), C.GoString(C.wva_last_error(e.h)))
 }
@@ -443,6 +451,50 @@ func (e *Engine) Resolve(r *Resident) (*config.AllocationSolution, error) {
 		return nil, e.fail("wva_resolve", rc)
 	}
 	return r.f.solution(win), nil
+}
+
+// ResolveScenarios is Resolve under len(loads) arrival-rate scenarios in one call (wva_resolve_scenarios): forecast
+// peaks, load percentiles, "what at 2x traffic".  loads[l] maps server names to scenario l's ArrivalRate (req/min);
+// a server missing from it keeps its resident rate.  Solution l equals UpdateLoad(arrival rates of loads[l]) +
+// Resolve, but the resident fleet keeps its own load, and Summarize has nothing to report until the next solve.
+func (e *Engine) ResolveScenarios(r *Resident, loads []map[string]float32) ([]*config.AllocationSolution, error) {
+	f := r.f
+	L, S := len(loads), len(f.serverNames)
+	if L == 0 {
+		return nil, nil
+	}
+	rows := make([]float32, L*S)
+	for l, ld := range loads {
+		row := rows[l*S : (l+1)*S]
+		copy(row, f.arrival)
+		for s, name := range f.serverNames {
+			if v, ok := ld[name]; ok {
+				row[s] = v
+			}
+		}
+	}
+	var pin runtime.Pinner
+	defer pin.Unpin()
+	pr := f32p(rows)
+	pin.Pin(unsafe.Pointer(pr))
+	win, cwin := newAllocs(L*S, &pin)
+	e.mu.Lock()
+	defer e.mu.Unlock()
+	if rc := C.wva_resolve_scenarios(e.h, C.int32_t(L), pr, nil, &cwin); rc != C.WVA_OK {
+		return nil, e.fail("wva_resolve_scenarios", rc)
+	}
+	out := make([]*config.AllocationSolution, L)
+	for l := range out {
+		sol := f.solution(win.slice(l*S, (l+1)*S))
+		for s, name := range f.serverNames { // the solution reports the load it was sized for
+			if d, ok := sol.Spec[name]; ok {
+				d.Load.ArrivalRate = rows[l*S+s]
+				sol.Spec[name] = d
+			}
+		}
+		out[l] = sol
+	}
+	return out, nil
 }
 
 // ---- System.AllocateByType + Solver.Solve's diffs ---------------------------------------------------------

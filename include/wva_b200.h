@@ -314,6 +314,20 @@ int wva_update_load(wva_handle *h, const float *arrival_rpm, const int32_t *in_t
                     const int32_t *out_tokens);
 /* wva_solve on the resident fleet. */
 int wva_resolve(wva_handle *h, wva_allocs *candidates, wva_allocs *winners);
+/* The reconcile of wva_resolve, repeated for n_scen arrival-rate columns of the resident fleet
+ * (forecast peaks, load percentiles, "what at 2x traffic").
+ *   arrival_rpm [n_scen * S]  row l = ServerLoadSpec.ArrivalRate of every server in scenario l (req/min)
+ *   candidates  [n_scen * S * A], index (l*S + s)*A + a; may be NULL
+ *   winners     [n_scen * S],     index l*S + s
+ * Scenario l's records are bit-identical to wva_update_load(arrival_rpm = row l) + wva_resolve, in unlimited and
+ * limited mode, and the call fails with the code wva_resolve would return for some scenario.  Only the arrival rate
+ * varies: QueueAnalyzer.Size never reads it, so each candidate is sized once and only CreateAllocation's per-load
+ * steps and final Analyze run per scenario.  The resident fleet (its load columns included) is not changed, but the
+ * most recent solution is cleared as by wva_update_load; wva_last_kernel_ms / wva_last_device_ms cover this call.
+ * WVA_ERR_BAD_ARG for n_scen < 1 or a NULL arrival_rpm / winners; WVA_ERR_UNSUPPORTED for n_scen > 65535 or
+ * n_scen * S * A > 2^31 - 1 (the kernels' index range). */
+int wva_resolve_scenarios(wva_handle *h, int32_t n_scen, const float *arrival_rpm, wva_allocs *candidates,
+                          wva_allocs *winners);
 
 /* ---- device-resident variants (used by the multi-GPU driver and bench) --- */
 

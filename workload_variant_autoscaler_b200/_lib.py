@@ -40,6 +40,7 @@ EXPORTS = (
     "wva_grid_solve_device", "wva_resolve_device", "wva_stream", "wva_synchronize", "wva_launch_count",
     "wva_last_kernel_ms", "wva_last_device_ms", "wva_summarize", "wva_solve_greedy", "wva_mm1k_solve",
     "wva_xchg_create", "wva_xchg_open", "wva_xchg_publish", "wva_xchg_error", "wva_xchg_destroy",
+    "wva_resolve_scenarios",
 )
 
 _lib = None
@@ -72,6 +73,7 @@ def lib():
         ("wva_upload", [vp, C.POINTER(_abi.FleetC)]),
         ("wva_update_load", [vp, f32p, i32p, i32p]),
         ("wva_resolve", [vp, C.POINTER(_abi.AllocsC), C.POINTER(_abi.AllocsC)]),
+        ("wva_resolve_scenarios", [vp, i32, f32p, C.POINTER(_abi.AllocsC), C.POINTER(_abi.AllocsC)]),
         ("wva_grid_solve_device", [vp, C.POINTER(_abi.GridC), C.POINTER(_abi.AllocsC)]),
         ("wva_resolve_device", [vp, C.POINTER(_abi.AllocsC)]),
         ("wva_synchronize", [vp]),

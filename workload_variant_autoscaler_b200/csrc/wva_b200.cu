@@ -86,14 +86,18 @@ struct HostFleet {
     int saturation_policy = 0;
     wva_tunables tun{10, 0.1f};
 
+    // the gates of pair_class that do not read the arrival rate
+    bool rate_free_gates(int s, int a, bool honour_keep) const {
+        if (honour_keep && srv_keep_acc[s] && srv_cur_acc[s] != WVA_ACC_NONE && srv_cur_acc[s] != a) return false;
+        if (srv_in_tokens[s] < 0 || srv_out_tokens[s] < 0) return false;
+        const int m = srv_model[s];
+        if (m < 0 || m >= M) return false;
+        if (!perf_present[(size_t)m * A + a]) return false;
+        return srv_has_target[s] != 0;
+    }
     // gates of CreateAllocation + candidate rule (mirrors pair_class on the device)
     int pair_class(int s, int a, bool honour_keep) const {
-        if (honour_keep && srv_keep_acc[s] && srv_cur_acc[s] != WVA_ACC_NONE && srv_cur_acc[s] != a) return 0;
-        if (srv_arrival_rpm[s] < 0.0f || srv_in_tokens[s] < 0 || srv_out_tokens[s] < 0) return 0;
-        const int m = srv_model[s];
-        if (m < 0 || m >= M) return 0;
-        if (!perf_present[(size_t)m * A + a]) return 0;
-        if (!srv_has_target[s]) return 0;
+        if (srv_arrival_rpm[s] < 0.0f || !rate_free_gates(s, a, honour_keep)) return 0;
         if (srv_arrival_rpm[s] == 0.0f || srv_out_tokens[s] == 0) return PAIR_ZERO;
         return PAIR_LOAD;
     }
@@ -137,6 +141,13 @@ struct wva_handle {
     DevBuf d_cand_pair, d_cand_N;
     DevBuf d_sz_tab, d_sz_ls, d_sz_off, d_sz_state, d_sz_req, d_sz_sort;
     PinBuf sz_pin;
+    // wva_resolve_scenarios: its own candidate list and tables (the list can differ from the size path's), cached
+    // while the token statistics and the set of servers loaded in some scenario stay the same
+    uint64_t scen_epoch = ~0ull;
+    std::vector<uint8_t> scen_loaded;
+    std::vector<int> scen_pair, scen_N;
+    int scen_Nmax = 0;
+    DevBuf d_scen_pair, d_scen_N, d_scen_tab, d_scen_ls, d_scen_off, d_scen_rpm;
 
     // grid path caches
     uint64_t grid_epoch = ~0ull;
@@ -432,6 +443,38 @@ int ensure_scratch(wva_handle* h, int Nmax, int ratio, size_t* slot_doubles, int
 }
 
 // ---- size path (K1) ---------------------------------------------------------
+// Keep a candidate list (pair ids sorted by descending N; Ns indexed by pair id) on the host and the device, and build
+// one shared-format service-rate table per candidate (N entries).
+int upload_size_list(wva_handle* h, const std::vector<int>& pairs, const std::vector<int>& Ns, std::vector<int>& cand_pair,
+                     std::vector<int>& cand_N, int& Nmax, DevBuf& d_pair, DevBuf& d_N, DevBuf& d_off, DevBuf& d_tab,
+                     DevBuf& d_ls) {
+    const int n = (int)pairs.size();
+    cand_pair = pairs;
+    cand_N.resize(n);
+    for (int j = 0; j < n; ++j) cand_N[j] = Ns[pairs[j]];
+    Nmax = n ? cand_N[0] : 1;
+    if (n) {
+        CK(d_pair.ensure(sizeof(int) * n));
+        CK(d_N.ensure(sizeof(int) * n));
+        CK(cudaMemcpyAsync(d_pair.p, cand_pair.data(), sizeof(int) * n, cudaMemcpyHostToDevice, h->stream));
+        CK(cudaMemcpyAsync(d_N.p, cand_N.data(), sizeof(int) * n, cudaMemcpyHostToDevice, h->stream));
+        // one shared-format service-rate table per candidate (N entries), cached until the token
+        // statistics or the fleet change
+        std::vector<long long> off(n + 1, 0);
+        for (int j = 0; j < n; ++j) off[j + 1] = off[j] + cand_N[j];
+        CK(d_off.ensure(sizeof(long long) * (n + 1)));
+        CK(d_tab.ensure(sizeof(double) * 4 * (size_t)off[n] + 1024));
+        CK(d_ls.ensure(sizeof(float) * ((size_t)off[n] + n + 1)));
+        CK(cudaMemcpyAsync(d_off.p, off.data(), sizeof(long long) * (n + 1), cudaMemcpyHostToDevice, h->stream));
+        build_pair_tables<<<n, 128, 0, h->stream>>>(h->df, (const int*)d_pair.p, (const long long*)d_off.p,
+                                                    (const int*)d_N.p, n, (double*)d_tab.p, (float*)d_ls.p, nullptr, 0,
+                                                    nullptr);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    return WVA_OK;
+}
+
 int prepare_size(wva_handle* h) {
     if (h->size_epoch == h->epoch_tokens) return WVA_OK;
     const HostFleet& hf = h->hf;
@@ -447,30 +490,9 @@ int prepare_size(wva_handle* h) {
                 pairs.push_back(s * A + a);
             }
     std::stable_sort(pairs.begin(), pairs.end(), [&](int x, int y) { return Ns[x] > Ns[y]; });
-    const int n = (int)pairs.size();
-    h->cand_pair = pairs;
-    h->cand_N.resize(n);
-    for (int j = 0; j < n; ++j) h->cand_N[j] = Ns[pairs[j]];
-    h->size_Nmax = n ? h->cand_N[0] : 1;
-    if (n) {
-        CK(h->d_cand_pair.ensure(sizeof(int) * n));
-        CK(h->d_cand_N.ensure(sizeof(int) * n));
-        CK(cudaMemcpyAsync(h->d_cand_pair.p, h->cand_pair.data(), sizeof(int) * n, cudaMemcpyHostToDevice, h->stream));
-        CK(cudaMemcpyAsync(h->d_cand_N.p, h->cand_N.data(), sizeof(int) * n, cudaMemcpyHostToDevice, h->stream));
-        // one shared-format service-rate table per candidate (N entries), cached until the token
-        // statistics or the fleet change
-        std::vector<long long> off(n + 1, 0);
-        for (int j = 0; j < n; ++j) off[j + 1] = off[j] + h->cand_N[j];
-        CK(h->d_sz_off.ensure(sizeof(long long) * (n + 1)));
-        CK(h->d_sz_tab.ensure(sizeof(double) * 4 * (size_t)off[n] + 1024));
-        CK(h->d_sz_ls.ensure(sizeof(float) * ((size_t)off[n] + n + 1)));
-        CK(cudaMemcpyAsync(h->d_sz_off.p, off.data(), sizeof(long long) * (n + 1), cudaMemcpyHostToDevice, h->stream));
-        build_pair_tables<<<n, 128, 0, h->stream>>>(h->df, (const int*)h->d_cand_pair.p, (const long long*)h->d_sz_off.p,
-                                                    (const int*)h->d_cand_N.p, n, (double*)h->d_sz_tab.p,
-                                                    (float*)h->d_sz_ls.p, nullptr, 0, nullptr);
-        h->launches++;
-        CK(cudaGetLastError());
-    }
+    int rc = upload_size_list(h, pairs, Ns, h->cand_pair, h->cand_N, h->size_Nmax, h->d_cand_pair, h->d_cand_N,
+                              h->d_sz_off, h->d_sz_tab, h->d_sz_ls);
+    if (rc) return rc;
     h->size_epoch = h->epoch_tokens;
     return WVA_OK;
 }
@@ -481,7 +503,10 @@ int size_depth_for(int n) {
     if (const char* e = getenv("WVA_SIZE_DEPTH")) d = atoi(e);
     return std::min(std::max(d, 1), kSzMaxDepth);
 }
-int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
+// `star` (wva_resolve_scenarios): the rounds stop at rateStar (sz2_advance<true>), the request block holds at least
+// min_cap slots, and *star receives the rounds' arguments for the scenario round that follows.
+int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n, const double* tab, const long long* tab_off,
+                    const float* ls, Sz2Args* star = nullptr, size_t min_cap = 0) {
     const int D = size_depth_for(n);
     int size_rev = 1;  // solver returns to the block vote after a per-step excursion (0 = stays on the per-step path)
     if (const char* e = getenv("WVA_SIZE_REV")) size_rev = atoi(e);
@@ -500,7 +525,7 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
     int dbg_round = -1;  // diagnostics: record per-request SM cycles of this round's sz2_solve (wva_dbg_read_size)
     if (const char* e = getenv("WVA_SIZE_DBG_ROUND")) dbg_round = atoi(e);
     const size_t per_cand = 2 * ((size_t)(1 << D) - 1 + 2);  // two searches: a tree each, plus the two end points
-    const size_t cap = per_cand * (size_t)n;                 // requests per round, worst case
+    const size_t cap = std::max(per_cand * (size_t)n, min_cap);  // requests per round, worst case
     const size_t n2 = 2 * (size_t)n;
     // state block
     size_t o = 0;
@@ -516,6 +541,7 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
     o = 0;
     const size_t r_id = take(4 * cap), r_lam = take(4 * cap), r_key = take(cap), r_out = take(16 * cap), r_bail = take(cap),
                  r_cnt = take(16);
+    const size_t r_scen = star ? take(4 * cap) : 0;
     CK(h->d_sz_req.ensure(o));
     char* rp = (char*)h->d_sz_req.p;
     // sort workspace
@@ -534,9 +560,9 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
     g.cand_N = sa.cand_N;
     g.n_cand = n;
     g.depth = D;
-    g.tab = (const double*)h->d_sz_tab.p;
-    g.tab_off = (const long long*)h->d_sz_off.p;
-    g.ls = (const float*)h->d_sz_ls.p;
+    g.tab = tab;
+    g.tab_off = tab_off;
+    g.ls = ls;
     g.xmin = (float*)(sp + o_xmin); g.xmax = (float*)(sp + o_xmax); g.xs = (float*)(sp + o_xs);
     g.sst = (uint8_t*)(sp + o_sst); g.inc = (uint8_t*)(sp + o_inc); g.iter = (uint8_t*)(sp + o_iter);
     g.ind = (int8_t*)(sp + o_ind); g.slot = (int*)(sp + o_slot);
@@ -548,10 +574,12 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
     g.req_id = (unsigned*)(rp + r_id); g.req_lam = (float*)(rp + r_lam); g.req_key = (uint8_t*)(rp + r_key);
     g.req_out = (float4*)(rp + r_out); g.req_bail = (uint8_t*)(rp + r_bail);
     g.n_req = (unsigned*)(rp + r_cnt); g.n_live = g.n_req + 1;
+    g.req_scen = star ? (int*)(rp + r_scen) : nullptr;
     g.ws.order = (unsigned*)(wp + w_order); g.ws.items = (unsigned long long*)(wp + w_items);
     g.ws.items_sorted = (unsigned long long*)(wp + w_sorted); g.ws.item_count = (unsigned*)(wp + w_cnt);
     g.cand = sa.cand;
     g.fb_count = sa.fb_count; g.fb_list = sa.fb_list; g.fb_cap = sa.fb_cap;
+    g.scen_rpm = sa.scen_rpm; g.n_scen = sa.n_scen;
 
     const unsigned nb = (unsigned)((n + 255) / 256);
     const unsigned cks = (unsigned)chunks, items_blocks = (unsigned)((max_items + 255) / 256),
@@ -567,7 +595,8 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
     for (int round = 0; round < max_rounds; round += group) {
         for (int r = 0; r < group; ++r) {
             sz2_round_reset<<<3, 256, 0, h->stream>>>(g);
-            sz2_advance<<<nb, 256, 0, h->stream>>>(g);
+            if (star) sz2_advance<true><<<nb, 256, 0, h->stream>>>(g);
+            else sz2_advance<false><<<nb, 256, 0, h->stream>>>(g);
             sz2_sort_local<<<cks, kSortThreads, 0, h->stream>>>(g);
             ws_items_scan<<<1, 256, 0, h->stream>>>(g.ws);
             ws_items_scatter<<<items_blocks, 256, 0, h->stream>>>(g.ws);
@@ -588,6 +617,10 @@ int run_size_rounds(wva_handle* h, const SizeArgs& sa, int n) {
         if (*pin == 0) break;
     }
     CK(cudaGetLastError());
+    if (star) {
+        g.dbg = nullptr;
+        *star = g;
+    }
     return WVA_OK;
 }
 
@@ -601,7 +634,7 @@ int enqueue_size(wva_handle* h, const AllocCols& cand, const AllocCols* winners)
     const int n_pairs = hf.S * hf.A;
     const int n = (int)h->cand_pair.size();
     if (n_pairs > 0) {
-        trivial_kernel<<<(n_pairs + 255) / 256, 256, 0, h->stream>>>(h->df, cand);
+        trivial_kernel<<<(n_pairs + 255) / 256, 256, 0, h->stream>>>(h->df, cand, nullptr);
         h->launches++;
     }
     SizeArgs g{};
@@ -614,6 +647,7 @@ int enqueue_size(wva_handle* h, const AllocCols& cand, const AllocCols* winners)
     CK(h->d_fb_list.ensure(sizeof(int) * std::max(n, 1)));
     g.fb_list = (int*)h->d_fb_list.p;
     g.fb_cap = std::max(n, 1);
+    g.n_scen = 1;
     CK(cudaEventRecord(h->ev_k0, h->stream));
     int small_max = 1024;  // up to here a warp per candidate beats rounds (the GPU is mostly empty either way)
     if (const char* e = getenv("WVA_SIZE_SMALL_MAX")) small_max = atoi(e);
@@ -622,7 +656,8 @@ int enqueue_size(wva_handle* h, const AllocCols& cand, const AllocCols* winners)
                                                                           (const long long*)h->d_sz_off.p);
         h->launches++;
     } else if (n > 0) {
-        rc = run_size_rounds(h, g, n);
+        rc = run_size_rounds(h, g, n, (const double*)h->d_sz_tab.p, (const long long*)h->d_sz_off.p,
+                             (const float*)h->d_sz_ls.p);
         if (rc) return rc;
     }
     CK(cudaEventRecord(h->ev_k1, h->stream));
@@ -1145,10 +1180,12 @@ void block_to_cands(const void* host_block, const Block& b, std::vector<HostCand
         c.max_rate = ((const float*)(p + b.off_rate))[i];
     }
 }
-void cands_to_abi(const std::vector<HostCand>& v, wva_allocs* out) {
+// writes v into records at .. at + v.size() - 1 of out
+void cands_to_abi(const std::vector<HostCand>& v, wva_allocs* out, size_t at = 0) {
     if (!out) return;
-    for (size_t i = 0; i < v.size(); ++i) {
-        const HostCand& c = v[i];
+    for (size_t k = 0; k < v.size(); ++k) {
+        const HostCand& c = v[k];
+        const size_t i = at + k;
         if (out->feasible) out->feasible[i] = c.feasible;
         if (out->acc) out->acc[i] = c.acc;
         if (out->replicas) out->replicas[i] = c.replicas;
@@ -1218,6 +1255,149 @@ int run_greedy_host(wva_handle* h, wva_allocs* candidates, wva_allocs* winners) 
         h->last_cost[s] = win[s].cost;
     }
     h->last_kind = 2;
+    return WVA_OK;
+}
+
+// ---- scenarios (wva_resolve_scenarios, DESIGN §3.8) --------------------------------------------------------------
+// Candidate list: every pair that passes the gates of CreateAllocation that do not read the arrival rate, has
+// out_tokens > 0, and carries load (a rate neither == 0 nor < 0, NaN included) in at least one scenario.  That is the
+// union over the scenarios of the lists prepare_size would build.
+int prepare_scenarios(wva_handle* h, int L, const float* rpm) {
+    const HostFleet& hf = h->hf;
+    const int A = hf.A, S = hf.S;
+    // the list is a function of the token epoch and of which servers carry load in some scenario
+    std::vector<uint8_t> loaded(S, 0);
+    for (int s = 0; s < S; ++s)
+        for (int l = 0; l < L && !loaded[s]; ++l) {
+            const float r = rpm[(size_t)l * S + s];
+            loaded[s] = !(r == 0.0f) && !(r < 0.0f);
+        }
+    if (h->scen_epoch == h->epoch_tokens && loaded == h->scen_loaded) return WVA_OK;
+    std::vector<int> pairs;
+    std::vector<int> Ns((size_t)S * A, 0);
+    for (int s = 0; s < S; ++s) {
+        if (hf.srv_out_tokens[s] <= 0 || !loaded[s]) continue;
+        for (int a = 0; a < A; ++a)
+            if (hf.rate_free_gates(s, a, true)) {
+                const int N = hf.pair_batch(s, a);
+                if (N > (1 << 20)) return h->fail(WVA_ERR_UNSUPPORTED, "batch size above 2^20");
+                Ns[(size_t)s * A + a] = N;
+                pairs.push_back(s * A + a);
+            }
+    }
+    std::stable_sort(pairs.begin(), pairs.end(), [&](int x, int y) { return Ns[x] > Ns[y]; });
+    int rc = upload_size_list(h, pairs, Ns, h->scen_pair, h->scen_N, h->scen_Nmax, h->d_scen_pair, h->d_scen_N,
+                              h->d_scen_off, h->d_scen_tab, h->d_scen_ls);
+    if (rc) return rc;
+    h->scen_loaded = loaded;
+    h->scen_epoch = h->epoch_tokens;
+    return WVA_OK;
+}
+
+// Size once (the rounds up to Analyze(lambda*)), then one round of final Analyze requests over (candidate, scenario),
+// then the per-scenario trivial / fallback / unlimited kernels.  The resident fleet is not modified.
+int run_scenarios(wva_handle* h, int L, const float* rpm, wva_allocs* candidates, wva_allocs* winners) {
+    const HostFleet& hf = h->hf;
+    if (!hf.unlimited)
+        for (int a = 0; a < hf.A; ++a)
+            if (hf.T <= 0 || hf.acc_type[a] < 0 || hf.acc_type[a] >= hf.T)
+                return h->fail(WVA_ERR_BAD_ARG, "limited mode needs a type id and a capacity for every accelerator");
+    int rc = prepare_scenarios(h, L, rpm);
+    if (rc) return rc;
+    rc = ensure_ctrl(h);
+    if (rc) return rc;
+    const size_t S = hf.S, A = hf.A;
+    const int n = (int)h->scen_pair.size();
+    const size_t n_req = (size_t)n * L;
+    const Block bc = block_layout((size_t)L * S * A), bw = block_layout((size_t)L * S);
+    CK(h->d_cand_block.ensure(bc.bytes + 16));
+    CK(h->d_win_block.ensure(bw.bytes + 16));
+    CK(h->d_scen_rpm.ensure(sizeof(float) * (size_t)L * S + 16));
+    const AllocCols dc = block_cols(h->d_cand_block.p, bc), dw = block_cols(h->d_win_block.p, bw);
+    const float* d_rpm = (const float*)h->d_scen_rpm.p;
+    CK(cudaEventRecord(h->ev_d0, h->stream));
+    if (S) CK(cudaMemcpyAsync(h->d_scen_rpm.p, rpm, sizeof(float) * (size_t)L * S, cudaMemcpyHostToDevice, h->stream));
+    if (S * A > 0) {
+        trivial_kernel<<<dim3((unsigned)((S * A + 255) / 256), (unsigned)L), 256, 0, h->stream>>>(h->df, dc, d_rpm);
+        h->launches++;
+    }
+    SizeArgs g{};
+    g.f = h->df;
+    g.cand_pair = (const int*)h->d_scen_pair.p;
+    g.cand_N = (const int*)h->d_scen_N.p;
+    g.n_cand = n;
+    g.cand = dc;
+    g.fb_count = (int*)h->d_ctrl.p + CTRL_FB_COUNT;
+    CK(h->d_fb_list.ensure(sizeof(int) * std::max<size_t>(n_req, 1)));
+    g.fb_list = (int*)h->d_fb_list.p;
+    g.fb_cap = (int)std::max<size_t>(n_req, 1);  // one entry per (candidate, scenario) at most
+    g.scen_rpm = d_rpm;
+    g.n_scen = L;
+    CK(cudaEventRecord(h->ev_k0, h->stream));
+    if (n > 0) {
+        SizeArgs rounds = g;
+        rounds.cand = AllocCols{};  // in STAR mode the rounds write no record
+        Sz2Args z;
+        rc = run_size_rounds(h, rounds, n, (const double*)h->d_scen_tab.p, (const long long*)h->d_scen_off.p,
+                             (const float*)h->d_scen_ls.p, &z, n_req);
+        if (rc) return rc;
+        z.cand = dc;
+        int size_rev = 1;
+        if (const char* e = getenv("WVA_SIZE_REV")) size_rev = atoi(e);
+        const size_t chunks = (n_req + kSortChunk - 1) / kSortChunk, max_items = (n_req + 31) / 32 + chunks;
+        const unsigned nb = (unsigned)((n_req + 255) / 256);
+        sz2_round_reset<<<3, 256, 0, h->stream>>>(z);
+        sz2_expand<<<nb, 256, 0, h->stream>>>(z);
+        sz2_sort_local<<<(unsigned)chunks, kSortThreads, 0, h->stream>>>(z);
+        ws_items_scan<<<1, 256, 0, h->stream>>>(z.ws);
+        ws_items_scatter<<<(unsigned)((max_items + 255) / 256), 256, 0, h->stream>>>(z.ws);
+        const unsigned solve_blocks = (unsigned)((max_items * 32 + 255) / 256);
+        if (size_rev) sz2_solve<1><<<solve_blocks, 256, 0, h->stream>>>(z);
+        else sz2_solve<0><<<solve_blocks, 256, 0, h->stream>>>(z);
+        sz2_consume<<<nb, 256, 0, h->stream>>>(z);
+        h->launches += 7;
+    }
+    CK(cudaEventRecord(h->ev_k1, h->stream));
+    if (n > 0) {
+        size_t slot_doubles;
+        int Kmax;
+        rc = ensure_scratch(h, h->scen_Nmax, hf.tun.max_queue_to_batch_ratio, &slot_doubles, &Kmax);
+        if (rc) return rc;
+        size_fallback<<<kFbBlocks, kFbThreads, 0, h->stream>>>(g, (double*)h->d_scratch.p, slot_doubles, Kmax,
+                                                               (int*)h->d_ctrl.p + CTRL_FB_STATUS);
+        h->launches++;
+    }
+    if (S > 0) {  // also assigns value = transition penalty, which the greedy pass reads
+        unlimited_kernel<<<dim3((unsigned)((S + 127) / 128), (unsigned)L), 128, 0, h->stream>>>(h->df, dc, dw);
+        h->launches++;
+    }
+    CK(cudaGetLastError());
+    const bool want_cand = candidates || !hf.unlimited, want_win = hf.unlimited;
+    CK(h->out_stage.ensure(align_up(bc.bytes) + align_up(bw.bytes) + 256));
+    char* hs = (char*)h->out_stage.p;
+    if (want_cand && bc.bytes) CK(cudaMemcpyAsync(hs, h->d_cand_block.p, bc.bytes, cudaMemcpyDeviceToHost, h->stream));
+    if (want_win && bw.bytes)
+        CK(cudaMemcpyAsync(hs + align_up(bc.bytes), h->d_win_block.p, bw.bytes, cudaMemcpyDeviceToHost, h->stream));
+    int* ctrl_host = (int*)(hs + align_up(bc.bytes) + align_up(bw.bytes));
+    CK(cudaMemcpyAsync(ctrl_host, h->d_ctrl.p, CTRL_INTS * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    rc = finish_timing(h);
+    if (rc) return rc;
+    rc = check_fallback_status(h, ctrl_host, (long long)n_req + 1);
+    if (rc) return rc;
+    if (hf.unlimited) {
+        scatter_block(hs, bc, candidates);
+        scatter_block(hs + align_up(bc.bytes), bw, winners);
+        return WVA_OK;
+    }
+    // limited mode: SolveGreedy once per scenario (it never reads the arrival rate)
+    std::vector<HostCand> all, cand, win(S);
+    block_to_cands(hs, bc, all);
+    for (int l = 0; l < L; ++l) {
+        cand.assign(all.begin() + (size_t)l * S * A, all.begin() + (size_t)(l + 1) * S * A);
+        GreedySolver(hf, cand, win).run();
+        cands_to_abi(cand, candidates, (size_t)l * S * A);
+        cands_to_abi(win, winners, (size_t)l * S);
+    }
     return WVA_OK;
 }
 
@@ -1503,6 +1683,17 @@ int wva_resolve(wva_handle* h, wva_allocs* candidates, wva_allocs* winners) {
     const int rc = run_size_host(h, candidates, winners);
     if (rc == WVA_OK) h->last_kind = 1;
     return rc;
+}
+
+int wva_resolve_scenarios(wva_handle* h, int32_t n_scen, const float* arrival_rpm, wva_allocs* candidates,
+                          wva_allocs* winners) {
+    if (!h || n_scen < 1 || !arrival_rpm || !winners) return WVA_ERR_BAD_ARG;
+    CK(cudaSetDevice(h->device));
+    if (!h->resident) return h->fail(WVA_ERR_STATE, "no resident fleet (call wva_upload first)");
+    h->last_kind = 0;  // like wva_update_load: the scenarios are not a solution of the resident fleet
+    if (n_scen > 65535 || (long long)n_scen * h->hf.S * h->hf.A > 0x7fffffffll)
+        return h->fail(WVA_ERR_UNSUPPORTED, "n_scen above 65535 or n_scen * S * A above 2^31 - 1");
+    return run_scenarios(h, n_scen, arrival_rpm, candidates, winners);
 }
 
 int wva_solve(wva_handle* h, const wva_fleet* fleet, wva_allocs* candidates, wva_allocs* winners) {

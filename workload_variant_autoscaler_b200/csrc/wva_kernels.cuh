@@ -8,8 +8,8 @@
 //   sz2_* kernels  K1   (wva_size.cuh) CreateAllocation per (server, acc) candidate as rounds of sorted solve
 //                       batches with speculative bisection trees
 //   size_fallback       stored-vector re-run of candidates that bailed
-//   trivial_kernel      nil / zero-load candidates
-//   unlimited_kernel    Server.Calculate value + SolveUnlimited argmin per server
+//   trivial_kernel      nil / zero-load candidates (per scenario for wva_resolve_scenarios)
+//   unlimited_kernel    Server.Calculate value + SolveUnlimited argmin per server (and scenario)
 //   sweep_kernel        Analyze over a rate sweep per (server, acc)
 //   sweep_fallback      stored-vector re-run of sweep points that bailed
 #pragma once
@@ -1471,15 +1471,17 @@ struct SizeArgs {
     const int* cand_pair;  // [n_cand] pair ids sorted by descending N
     const int* cand_N;     // [n_cand]
     int n_cand;
-    AllocCols cand;        // [S*A]
+    AllocCols cand;        // [n_scen*S*A]
     int* fb_count;
-    int* fb_list;          // candidate indices that bailed
+    int* fb_list;          // entries j * n_scen + l: candidate j bailed under scenario l
     int fb_cap;
+    const float* scen_rpm;  // [n_scen*S] arrival columns of wva_resolve_scenarios; NULL = the fleet's own
+    int n_scen;             // 1 without scenarios
 };
 
 // Stored-vector re-run of bailed candidates (slot k handles list entries k, k+n_slots, ..).
 __global__ void size_fallback(SizeArgs g, double* scratch, size_t slot_doubles, int Kmax, int* fb_status) {
-    const DevFleet& f = g.f;
+    DevFleet f = g.f;
     const int n_slots = gridDim.x * blockDim.x;
     const int slot = blockIdx.x * blockDim.x + threadIdx.x;
     int n = *g.fb_count;
@@ -1487,7 +1489,9 @@ __global__ void size_fallback(SizeArgs g, double* scratch, size_t slot_doubles, 
     double* p = scratch + (size_t)slot * slot_doubles;
     float* sr = (float*)(p + Kmax + 1);
     for (int k = slot; k < n; k += n_slots) {
-        const int j = g.fb_list[k];
+        const int e = g.fb_list[k];
+        const int j = e / g.n_scen, l = e - j * g.n_scen;
+        if (g.scen_rpm) f.srv_arrival_rpm = g.scen_rpm + (size_t)l * f.S;
         const int pair = g.cand_pair[j];
         const int s = pair / f.A, a = pair % f.A;
         StoredSolver sv;
@@ -1504,7 +1508,7 @@ __global__ void size_fallback(SizeArgs g, double* scratch, size_t slot_doubles, 
             atomicExch(fb_status, sv.bail);
             c = cand_nil();
         }
-        store_cand(g.cand, pair, c);
+        store_cand(g.cand, (size_t)l * f.S * f.A + pair, c);
     }
 }
 
@@ -1540,27 +1544,31 @@ __global__ void __launch_bounds__(256) ws_items_scatter(SortWs ws) {
 }
 
 
-// nil and zero-load candidates (everything the size kernel does not own).
-__global__ void trivial_kernel(DevFleet f, AllocCols cand) {
+// nil and zero-load candidates (everything the size kernel does not own).  blockIdx.y = scenario l of
+// wva_resolve_scenarios: row l of scen_rpm replaces the fleet's arrival column and the records go to block l.
+__global__ void trivial_kernel(DevFleet f, AllocCols cand, const float* scen_rpm) {
     const int pair = blockIdx.x * blockDim.x + threadIdx.x;
     if (pair >= f.S * f.A) return;
+    if (scen_rpm) f.srv_arrival_rpm = scen_rpm + (size_t)blockIdx.y * f.S;
     const int s = pair / f.A, a = pair % f.A;
     const int cls = pair_class(f, s, a, true);
     if (cls == PAIR_LOAD) return;
     Cand c = cand_nil();
     if (cls == PAIR_ZERO) c = zero_load_alloc(f, s, a);
-    store_cand(cand, pair, c);
+    store_cand(cand, (size_t)blockIdx.y * f.S * f.A + pair, c);
 }
 
 // Server.Calculate's value (server.go:60-63) + SolveUnlimited (solver.go:63-79):
-// one thread per server; strict '<' from MaxFloat32, lowest accelerator id wins ties.
+// one thread per server; strict '<' from MaxFloat32, lowest accelerator id wins ties.  blockIdx.y = scenario
+// (candidate block y, winner block y); nothing here reads the arrival rate.
 __global__ void unlimited_kernel(DevFleet f, AllocCols cand, AllocCols winners) {
     const int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= f.S) return;
     float min_val = 3.40282346638528859811704183484516925440e+38f;
     Cand best = cand_nil();
+    const size_t scen = blockIdx.y;
     for (int a = 0; a < f.A; ++a) {
-        const size_t i = (size_t)s * f.A + a;
+        const size_t i = (scen * f.S + s) * f.A + a;
         if (!cand.feasible[i]) continue;
         Cand c = load_cand(cand, i);
         c.value = penalty_of(f, s, c);
@@ -1570,7 +1578,7 @@ __global__ void unlimited_kernel(DevFleet f, AllocCols cand, AllocCols winners) 
             best = c;
         }
     }
-    store_cand(winners, s, best);
+    store_cand(winners, scen * f.S + s, best);
 }
 
 // ---------------------------------------------------------------------------

@@ -49,6 +49,7 @@ struct Sz2Args {
     int* aslot;            // [n] request slot of the candidate's Analyze this round
     // requests of the current round
     unsigned* req_id;      // 4*j + kind (0 TTFT eval, 1 ITL eval, 2 Analyze(lambda*), 3 Analyze(final))
+    int* req_scen;         // scenario of a kind-3 request emitted by sz2_expand
     float* req_lam;
     uint8_t* req_key;
     float4* req_out;       // kinds 0/1: x = y; kinds 2/3: throughput, ttft, itl, rho
@@ -61,6 +62,8 @@ struct Sz2Args {
     int* fb_list;
     int fb_cap;
     unsigned* dbg;         // diagnostics (WVA_SIZE_DBG_ROUND): per slot {SM cycles, N, lambda bits, warp}, or NULL
+    const float* scen_rpm;  // wva_resolve_scenarios: [n_scen*S] arrival columns (sz2_expand / sz2_consume)
+    int n_scen;
 };
 
 __device__ __forceinline__ float sz_mid(float lo, float hi) { return __fmul_rn(0.5f, __fadd_rn(lo, hi)); }  // utils.go:55
@@ -110,6 +113,9 @@ __global__ void __launch_bounds__(256) sz2_init(Sz2Args g) {
 
 // Advance every candidate: consume last round's results (walking the midpoint trees with the reference's
 // comparisons), then emit this round's requests into consecutive slots.
+// STAR (wva_resolve_scenarios): stop after Analyze(lambda*) with rateStar in rate_star[j] and phase PH_DONE; nil and
+// bailed candidates only leave their phase behind (no record, no fallback entry): sz2_expand handles them per scenario.
+template <bool STAR>
 __global__ void __launch_bounds__(256) sz2_advance(Sz2Args g) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     const DevFleet& f = g.f;
@@ -216,7 +222,10 @@ __global__ void __launch_bounds__(256) sz2_advance(Sz2Args g) {
         } else if (ph == PH_WAIT_STAR) {
             const int slot = g.aslot[j];
             if (g.req_bail[slot]) ph = PH_BAIL;
-            else {
+            else if (STAR) {
+                g.rate_star[j] = g.req_out[slot].x;  // metrics.Throughput
+                ph = PH_DONE;
+            } else {
                 const float rate_star = g.req_out[slot].x;  // metrics.Throughput
                 const float total_rate = total_rate_of(f, s);  // allocation.go:134-141
                 long long nrep = go_f64_to_int(ceil(__ddiv_rn((double)total_rate, (double)rate_star)));
@@ -250,11 +259,13 @@ __global__ void __launch_bounds__(256) sz2_advance(Sz2Args g) {
                 ph = PH_DONE;
             }
         }
-        if (ph == PH_NIL) store_cand(g.cand, pair, cand_nil());
-        if (ph == PH_BAIL) {
-            const int k = atomicAdd(g.fb_count, 1);
-            if (k < g.fb_cap) g.fb_list[k] = j;
-            store_cand(g.cand, pair, cand_nil());
+        if (!STAR) {
+            if (ph == PH_NIL) store_cand(g.cand, pair, cand_nil());
+            if (ph == PH_BAIL) {
+                const int k = atomicAdd(g.fb_count, 1);
+                if (k < g.fb_cap) g.fb_list[k] = j;
+                store_cand(g.cand, pair, cand_nil());
+            }
         }
         g.phase[j] = (uint8_t)ph;
     }
@@ -394,6 +405,111 @@ __global__ void __launch_bounds__(256, 4) sz2_solve(Sz2Args g) {
         out = make_float4(m.throughput, m.ttft, m.avg_token_time, m.rho);
     }
     g.req_out[slot] = out;
+}
+
+// ---------------------------------------------------------------------------
+// wva_resolve_scenarios (DESIGN §3.8): after a STAR run of the rounds, rateStar (or nil / bail) per candidate does not
+// depend on the arrival rate; only CreateAllocation's per-load steps and its final Analyze do.  sz2_expand applies the
+// steps per (candidate, scenario) and emits one kind-3 request per survivor, sz2_sort_local / ws_items_* / sz2_solve
+// run that round unchanged, and sz2_consume writes the records into the scenario's block.
+// ---------------------------------------------------------------------------
+struct LoadStep {
+    long long nrep;
+    float cost, rate;
+};
+// allocation.go:134-153 with the arrival column of f (the expressions of sz2_advance's PH_WAIT_STAR)
+__device__ __forceinline__ LoadStep load_step(const DevFleet& f, int s, int a, float rate_star) {
+    LoadStep r;
+    const float total_rate = total_rate_of(f, s);
+    r.nrep = go_f64_to_int(ceil(__ddiv_rn((double)total_rate, (double)rate_star)));
+    const long long min_rep = f.srv_min_replicas[s];
+    if (r.nrep < min_rep) r.nrep = min_rep;
+    const long long total = (long long)num_instances(f, f.srv_model[s], a) * r.nrep;
+    r.cost = __fmul_rn(f.acc_cost[a], (float)total);
+    r.rate = __fdiv_rn(total_rate, (float)r.nrep);
+    return r;
+}
+
+// One thread per (candidate j, scenario l), t = j * n_scen + l: a candidate's requests take consecutive slots.
+__global__ void __launch_bounds__(256) sz2_expand(Sz2Args g) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int L = g.n_scen;
+    int j = 0, l = 0;
+    bool emit = false;
+    float lambda = 0.0f;
+    if (t < (long long)g.n_cand * L) {
+        j = (int)(t / L);
+        l = (int)(t - (long long)j * L);
+        DevFleet f = g.f;
+        f.srv_arrival_rpm = g.scen_rpm + (size_t)l * f.S;
+        const int pair = g.cand_pair[j], s = pair / f.A, a = pair % f.A;
+        if (pair_class(f, s, a, true) == PAIR_LOAD) {  // otherwise trivial_kernel owns the record
+            const int ph = g.phase[j];
+            if (ph == PH_DONE) {
+                const LoadStep st = load_step(f, s, a, g.rate_star[j]);
+                if (!(st.rate <= 0.0f || st.rate > g.rmax[j])) {  // Analyze: queueanalyzer.go:135-143
+                    emit = true;
+                    lambda = __fdiv_rn(st.rate, 1000.0f);
+                }
+            } else if (ph == PH_BAIL) {
+                const int k = atomicAdd(g.fb_count, 1);
+                if (k < g.fb_cap) g.fb_list[k] = (int)t;
+            }
+            if (!emit) store_cand(g.cand, (size_t)l * f.S * f.A + pair, cand_nil());
+        }
+    }
+    const int mine = emit ? 1 : 0;
+    int incl = mine;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int o = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += o;
+    }
+    const int warp_total = __shfl_sync(0xffffffffu, incl, 31);
+    unsigned warp_base = 0;
+    if (lane == 31 && warp_total > 0) warp_base = atomicAdd(g.n_req, (unsigned)warp_total);
+    warp_base = __shfl_sync(0xffffffffu, warp_base, 31);
+    if (!emit) return;
+    const unsigned slot = warp_base + (unsigned)(incl - mine);
+    const int N = g.cand_N[j], K = N + N * g.f.ratio;
+    const long long off = g.tab_off[j];
+    g.req_id[slot] = (unsigned)j * 4u + 3u;
+    g.req_scen[slot] = l;
+    g.req_lam[slot] = lambda;
+    g.req_key[slot] = (uint8_t)length_class(estimate_len(g.tab + 4 * off, g.ls + off + j, N, K, lambda, log2f(lambda),
+                                                         g.l2s0[j], g.l2sN[j], g.lsN[j]));
+}
+
+// One thread per request of sz2_expand's round: the record of PH_WAIT_FINAL, or a stored-vector fallback entry.
+__global__ void __launch_bounds__(256) sz2_consume(Sz2Args g) {
+    const unsigned slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot >= *g.n_req) return;
+    const int j = (int)(g.req_id[slot] >> 2), l = g.req_scen[slot];
+    DevFleet f = g.f;
+    f.srv_arrival_rpm = g.scen_rpm + (size_t)l * f.S;
+    const int pair = g.cand_pair[j], s = pair / f.A, a = pair % f.A;
+    const size_t out = (size_t)l * f.S * f.A + pair;
+    if (g.req_bail[slot]) {
+        const int k = atomicAdd(g.fb_count, 1);
+        if (k < g.fb_cap) g.fb_list[k] = j * g.n_scen + l;
+        store_cand(g.cand, out, cand_nil());
+        return;
+    }
+    const LoadStep st = load_step(f, s, a, g.rate_star[j]);
+    const float4 m = g.req_out[slot];
+    Cand c = cand_nil();
+    c.feasible = 1;
+    c.acc = a;
+    c.replicas = (int)st.nrep;
+    c.batch = g.cand_N[j];
+    c.cost = st.cost;
+    c.value = c.cost;
+    c.itl = m.z;
+    c.ttft = m.y;
+    c.rho = m.w;
+    c.max_rate = __fdiv_rn(g.rate_star[j], 1000.0f);
+    store_cand(g.cand, out, c);
 }
 
 // ---------------------------------------------------------------------------

@@ -154,6 +154,27 @@ class Engine:
         self._check(self._L.wva_resolve(self._h, C.byref(cc) if cc is not None else None, C.byref(wc)))
         return cand, win
 
+    def resolve_scenarios(self, arrival_rpm, want_candidates: bool = False):
+        """``resolve`` of the resident fleet under L arrival-rate scenarios in one call (``wva_resolve_scenarios``).
+
+        ``arrival_rpm`` is ``[L, S]``: row l is every server's arrival rate (req/min) in scenario l.  Returns
+        (candidates [L*S*A] | None, winners [L*S]); scenario l's block (records l*S*A.. / l*S..) equals
+        ``update_load(arrival_rpm=row l)`` + ``resolve()``.  The resident fleet keeps its own load columns."""
+        if self._n_servers is None:
+            raise WvaError(_abi.WVA_ERR_STATE, "no resident fleet (call upload or a solve first)")
+        a = np.ascontiguousarray(arrival_rpm, np.float32)
+        if a.ndim != 2 or a.shape[1] != self._n_servers:  # the C side reads exactly L * S entries
+            raise ValueError(f"arrival_rpm must have shape [L, {self._n_servers}] (one row per scenario, one column "
+                             f"per resident server), got shape {a.shape}")
+        n_scen, S = a.shape
+        cand = Allocs(n_scen * S * self._n_acc) if want_candidates else None
+        win = Allocs(n_scen * S)
+        wc = win.as_c()
+        cc = cand.as_c() if cand is not None else None
+        self._check(self._L.wva_resolve_scenarios(self._h, n_scen, _abi.ptr(a), C.byref(cc) if cc is not None else None,
+                                                  C.byref(wc)))
+        return cand, win
+
     def summarize(self, n_types: int) -> dict:
         """``System.AllocateByType`` (pkg/core/system.go:271-300) and ``CreateAllocationDiff`` per server
         (pkg/core/allocation.go:353-380) over the most recent solution of this engine.
